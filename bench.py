@@ -32,6 +32,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 LOGS = list(range(10, 21))
 BATCH = 4096
@@ -422,20 +423,43 @@ def run_ours(args, rank: int, world: int, local_rank: int):
             run_size(lg)
     barrier()
 
+    # --dump-outputs: the same seeded choice of whole transforms of every size in every run (2^19 elements per size, one
+    # transform at 2^20: 48 MiB for the default sweep), taken from rank 0's last timed step
+    dump_rows = {}
+    if args.dump_outputs and rank == 0:
+        pick = np.random.default_rng(1234)
+        dump_rows = {lg: torch.from_numpy(np.sort(pick.choice(BATCH, max(1, (1 << 19) >> lg), replace=False))).to(dev) for lg in logs}
+    dumped = {}
+
     sampler = ClockSampler(local_rank)
     sampler.start()
     ev = [[torch.cuda.Event(enable_timing=True) for _ in range(len(logs) + 1)] for _ in range(args.steps)]
+    begin = [row[:-1] for row in ev]  # size i of step s is timed from begin[s][i] to ev[s][i + 1]
     barrier()
     for s in range(args.steps):
         ev[s][0].record()
         for i, lg in enumerate(logs):
             run_size(lg)
             ev[s][i + 1].record()
+            if dump_rows and s == args.steps - 1:
+                # every size's output region lies inside the largest size's, so each output is sampled before the next size
+                # runs; the next size's window starts after the copy, which stays out of the timing
+                n = 1 << lg
+                dumped[lg] = dst[offs[lg]: offs[lg] + BATCH * n].view(BATCH, n).index_select(0, dump_rows[lg])
+                if i + 1 < len(logs):
+                    begin[s][i + 1] = torch.cuda.Event(enable_timing=True)
+                    begin[s][i + 1].record()
     barrier()
     clocks = sampler.stop()
     total_ms = ev[0][0].elapsed_time(ev[-1][-1])
-    per_ms = {lg: sum(ev[s][i].elapsed_time(ev[s][i + 1]) for s in range(args.steps)) / args.steps
+    if dump_rows:
+        total_ms -= sum(ev[-1][i].elapsed_time(begin[-1][i]) for i in range(1, len(logs)))
+    per_ms = {lg: sum(begin[s][i].elapsed_time(ev[s][i + 1]) for s in range(args.steps)) / args.steps
               for i, lg in enumerate(logs)}
+    if dumped:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for lg, rows in dumped.items():
+            np.save(os.path.join(args.dump_outputs, f"fft_f32_forward_log2n{lg}.npy"), torch.view_as_real(rows).cpu().numpy())
     # supplementary: per-size time from R back-to-back execs (amortises the ~10 us launch+drain of a single
     # exec, which is comparable to the whole transform time at N = 2^10..2^12)
     per_ms_rep = {}
@@ -823,7 +847,14 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="plain stream launches instead of CUDA-graph replay")
     ap.add_argument("--profile", action="store_true", help="short run for ncu: 1 warm-up, no e2e / cpu legs")
     ap.add_argument("--profile-cold", action="store_true", help="with --profile: no warm-up sweep at all (launch lists)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/fft_f32_forward_log2n<L>.npy: float32 (rows, 2^L, 2), "
+                         "the same seeded choice of whole transforms (rows) of every size in every run")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

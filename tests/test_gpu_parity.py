@@ -36,10 +36,25 @@ def planner(request, torch_cuda):
 
 
 def test_native_library_is_the_one_running(torch_cuda):
+    import os
+    import subprocess
+    import sys
+
+    from util import ROOT
+
     lib = rb.default_library()
     assert lib.path.endswith("rustfft_b200/libb200fft.so") and lib.device_count() >= 1
-    maps = open("/proc/self/maps").read()
-    assert "libb200fft.so" in maps and "libb200fft_emu" not in maps
+    # the mapping check runs in a process of its own: the CPU tests of the same session load the emulation library into this one
+    code = ("import rustfft_b200 as rb\n"
+            "lib = rb.default_library()\n"
+            "assert lib.path.endswith('rustfft_b200/libb200fft.so') and lib.device_count() >= 1\n"
+            "maps = open('/proc/self/maps').read()\n"
+            "assert 'libb200fft.so' in maps and 'libb200fft_emu' not in maps\n"
+            "print('NATIVE-OK')\n")
+    e = dict(os.environ)
+    e["PYTHONPATH"] = ROOT + os.pathsep + os.path.join(ROOT, "tests")
+    r = subprocess.run([sys.executable, "-c", code], env=e, capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0 and "NATIVE-OK" in r.stdout, r.stdout[-2000:] + r.stderr[-2000:]
 
 
 def test_accuracy_every_len_1_to_1000(planner):
